@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- GCUPS of the NW/SW fill+traceback hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c4|c5] [--pairs P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c4|c5] [--pairs P] [--dump-outputs DIR]
 
 --config c2 (default, the bench line): BASELINE.json configs[1] -- a synthetic batch of P (default 1 M) pairs,
 150 bp pattern x 1 kb text DNA, seed 481, scoring 1/-1/-1, global AND local, score + traceback.  One "step" =
@@ -32,6 +32,14 @@ one pass of the hot path over the batch in both modes.
 --config c4: one 100 kb x 100 kb pair, local, score + traceback (configs[3]).  --config c5: the reference's own
 16 x 100 kb input, all-vs-all score-only, hw3's affine scoring and hw2's linear scoring (configs[4]), pairs
 sharded over the ranks.  Same JSON shape; rooflines against the int32 lines.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the headline (device-resident) path returned in its last
+step as DIR/<name>.npy (float32 where every value is exact in it, else float64; at most DUMP_BYTES in all), so that two
+builds can be compared output for output on identical seeded inputs.  c2/c4: per mode the record fields <mode>_<field>
+of the pairs in pair_index (every pair when they fit, else a fixed seeded sample), and <mode>_ops: the op lists of the
+pairs in ops_pair_index as ASCII codes (M 77, D 68, I 73) in traceback order, one row per pair, zero-padded.
+c5: affine_pair_scores, affine_star_sums, affine_centre of all 120 pairs (with N > 1 the ranks' shards are summed into
+rank 0 after the timed steps).  c2 and c4 dump rank 0's own batch, which does not depend on N either.
 """
 import argparse
 import json
@@ -114,6 +122,48 @@ def bind_to_gpu_numa_node(index):
     except Exception:
         pass
     return None
+
+
+DUMP_BYTES = 64_000_000
+DUMP_OPS_PAIRS = 256                    # op lists per mode in a dump
+RECORD_FIELDS = ("score", "end_i", "end_j", "start_i", "start_j", "overlap", "n_ops")    # "path" names the kernel family, not a result
+
+
+def dump_pairs(n_pairs, n_txt_max):
+    """(pair_index, ops_pair_index) of a dump: every pair whose record fits the budget left by the op lists, else a fixed seeded
+    sample; the op lists of a fixed seeded sample of those."""
+    ops_bytes = 2 * DUMP_OPS_PAIRS * (M + n_txt_max) * 4
+    per_pair = 2 * len(RECORD_FIELDS) * 4 + (4 if n_pairs <= 1 << 24 else 8)
+    keep = (DUMP_BYTES - ops_bytes - 4096) // per_pair
+    rng = np.random.default_rng(0)
+    idx = np.arange(n_pairs) if n_pairs <= keep else np.sort(rng.choice(n_pairs, size=keep, replace=False))
+    ops_idx = np.sort(rng.choice(idx, size=min(DUMP_OPS_PAIRS, len(idx)), replace=False))
+    return idx, ops_idx
+
+
+def alignment_arrays(name, records, idx, ops):
+    """<name>_<field> of the records at idx, and <name>_ops: one zero-padded row of ASCII op codes per op list"""
+    out = {f"{name}_{f}": records[f][idx] for f in RECORD_FIELDS}
+    rows = np.zeros((len(ops), max([len(o) for o in ops] + [1])), dtype=np.uint8)
+    for r, o in enumerate(ops):
+        rows[r, :len(o)] = np.frombuffer(o, dtype=np.uint8)
+    out[f"{name}_ops"] = rows
+    return out
+
+
+def write_dump(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        v = a.astype(np.float32)
+        if not np.array_equal(v, a):
+            v = a.astype(np.float64)
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, v)
+        total += os.path.getsize(path)
+    if total > DUMP_BYTES:
+        raise RuntimeError(f"--dump-outputs wrote {total} bytes, more than {DUMP_BYTES}")
 
 
 def load_peaks():
@@ -274,11 +324,12 @@ def shm_path(tag):
 # ------------------------------------------------------------------------------------------------------------
 # config 2 / 3
 # ------------------------------------------------------------------------------------------------------------
-def device_arm(pkg, dev, pat, po, txt, to, steps, warmup, local_rank, seg_pairs=0):
-    """inputs resident in HBM; returns per-mode kernel times (sums over `steps`), the launches and the result arrays for checking.
+def device_arm(pkg, dev, pat, po, txt, to, steps, warmup, local_rank, seg_pairs=0, ops_pairs=()):
+    """inputs resident in HBM; returns per-mode kernel times (sums over `steps`), the launches, the result arrays for checking and the op
+    lists of ops_pairs, all of the last step.
     The two modes run one after the other, each with its own engine: a 1 M-pair record is 55 GB per mode (110 GB with 4-bit deltas)."""
     fill_ms = {0: 0.0, 1: 0.0}; tb_ms = {0: 0.0, 1: 0.0}; tot_ms = {0: 0.0, 1: 0.0}
-    check, launches, wall, fill_bytes = {}, 0, 0.0, 0
+    check, ops, launches, wall, fill_bytes = {}, {}, 0, 0.0, 0
     n = len(po) - 1
     sampler = ClockSampler(local_rank)
     for mode in (pkg.GLOBAL, pkg.LOCAL):
@@ -301,12 +352,13 @@ def device_arm(pkg, dev, pat, po, txt, to, steps, warmup, local_rank, seg_pairs=
         wall += time.perf_counter() - t0
         launches += eng.stats()["launches"] - l0
         check[mode] = eng.download(n)
+        ops[mode] = [eng.fetch_ops(int(q), check[mode]["n_ops"][q]) for q in ops_pairs]
         if mode == pkg.GLOBAL:
             fill_bytes = eng.stats()["fill_bytes"]
         eng.close()
     clocks = sampler.summary()
     return {"fill_ms": fill_ms, "tb_ms": tb_ms, "tot_ms": tot_ms, "wall": wall, "clocks": clocks, "launches": launches,
-            "check": check, "fill_bytes": fill_bytes}
+            "check": check, "ops": ops, "fill_bytes": fill_bytes}
 
 
 def bench_c2(args):
@@ -332,7 +384,8 @@ def bench_c2(args):
     cells_mode = n_pairs * M * N_TXT
 
     # ---- weak, device-resident: W warm-up steps, then exactly K timed steps ----
-    d = device_arm(pkg, dev, pat, po, txt, to, args.steps, args.warmup, local_rank, args.resident_seg_pairs)
+    dump_idx, dump_ops_idx = dump_pairs(n_pairs, N_TXT) if args.dump_outputs and rank == 0 else (None, ())
+    d = device_arm(pkg, dev, pat, po, txt, to, args.steps, args.warmup, local_rank, args.resident_seg_pairs, dump_ops_idx)
     fill_ms, tb_ms, tot_ms = d["fill_ms"], d["tb_ms"], d["tot_ms"]
     dev_s = max_over_ranks(sum(tot_ms.values()) * 1e-3)
     wall_dev = max_over_ranks(d["wall"])
@@ -565,6 +618,11 @@ def bench_c2(args):
                 "sw_tb_ms": tb_ms[1] / args.steps, "nw_gcups": gc(tot_ms[0]), "sw_gcups": gc(tot_ms[1]),
                 "frac_fill": roofline["frac_fill"], "frac_step": roofline["frac_step"],
                 "gpu_launches": d["launches"], "clocks": d["clocks"], "roofline": roofline, "cpu_baseline": cpu}
+        if args.dump_outputs:
+            arrays = {"pair_index": dump_idx, "ops_pair_index": dump_ops_idx}
+            for mode, name in ((pkg.GLOBAL, "global"), (pkg.LOCAL, "local")):
+                arrays.update(alignment_arrays(name, d["check"][mode], dump_idx, d["ops"][mode]))
+            write_dump(args.dump_outputs, arrays)
     dev.close()
     if rank == 0:
         print(json.dumps(line))
@@ -603,6 +661,7 @@ def bench_c4(args):
     clocks = sampler.summary()
     launches = eng.stats()["launches"] - l0
     res = eng.download(1)
+    res_ops = [eng.fetch_ops(0, res["n_ops"][0])] if args.dump_outputs else []
     res_host = pkg.pinned_empty(1, pkg.RESULT_DTYPE)
     eng.align_packed(pkg.LOCAL, pat, po, txt, to, *s, want_ops=True, results=res_host)
     dev.barrier()
@@ -638,6 +697,8 @@ def bench_c4(args):
                              "peak_source": "b2a_microbench_int16x2 kind 0 lane-instruction rate measured in this run, one int32 cell per lane (SURVEY 8d: half the s16x2 line)"},
                 "cpu_baseline": cpu}
         assert ok, "config 4 result differs from the oracle"
+        if args.dump_outputs:
+            write_dump(args.dump_outputs, {"pair_index": [0], "ops_pair_index": [0], **alignment_arrays("local", res, [0], res_ops)})
     eng.close()
     dev.close()
     if rank == 0:
@@ -652,7 +713,7 @@ def bench_c5(args):
     from __graft_entry__ import load_package
     pkg = load_package()
     from bioinformatics_algorithms_b200 import workload
-    from bioinformatics_algorithms_b200.sharding import max_over_ranks, sum_over_ranks, star_pair_range
+    from bioinformatics_algorithms_b200.sharding import max_over_ranks, sum_over_ranks, star_pair_range, reduce_star_sums
     dev = Dist()
     rank, world, local_rank = dev.rank, dev.world, dev.local_rank
     seqs = [x for _, x in workload.config5_shipped()]
@@ -677,6 +738,11 @@ def bench_c5(args):
     st = eng.stats()
     dev_s = max_over_ranks(k_ms * 1e-3)
     total_cells = sum_over_ranks(cells * args.steps)
+    if args.dump_outputs and world > 1:             # every rank: the dump holds all pairs' scores and the full sums whatever the GPU count
+        all_ps = np.zeros(len(ij), dtype=np.int64)
+        all_ps[first:first + count] = ps
+        ps, _ = reduce_star_sums(all_ps)
+        sums, centre = reduce_star_sums(sums)
     # hw2's linear scoring over the same pairs, score only
     pat, po = pkg.pack([seqs[i] for i, _ in mine]); txt, to = pkg.pack([seqs[j] for _, j in mine])
     eng.upload(pkg.GLOBAL, pat, po, txt, to, 1, -1, -1, score_only=True)
@@ -707,6 +773,8 @@ def bench_c5(args):
                              "linear_frac": cells * args.steps * 5.0 / (lin_ms * 1e-3) / 1e9 / gops0,
                              "peak_source": "b2a_microbench_int16x2 kind 0 lane-instruction rate measured in this run, one int32 cell per lane"},
                 "cpu_baseline": cpu}
+        if args.dump_outputs:
+            write_dump(args.dump_outputs, {"affine_pair_scores": ps, "affine_star_sums": sums, "affine_centre": [centre]})
     eng.close()
     dev.close()
     if rank == 0:
@@ -729,7 +797,12 @@ def main():
     ap.add_argument("--resident-seg-pairs", type=int, default=0, help="experiment: pairs per segment of the device-resident arm")
     ap.add_argument("--n-rate", type=float, default=0.0, help="c2 variant: fraction of pattern bases turned into 'N' (pairs holding one leave the 4-symbol s16x2 path)")
     ap.add_argument("--scoring", default="1,-1,-1", help="c2: match,mismatch,gap (SURVEY 8d also names 2,-3,-4: 4-bit deltas, twice the record)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path; the reference arm has none to dump")
 
     if args.impl == "reference":
         if env_int("RANK", 0) != 0:
