@@ -6,14 +6,16 @@
 // delta record yields in O(1) per cell (one 16-byte chunk load + a popcount prefix sum from the anchor).
 //
 // Shaped for a WARP of 32 independent walks, where anything that is rare per thread happens almost every
-// iteration somewhere in the warp:
-//   * the general step is uniform and branch-free: both rows are re-sought every step (the chunk of the
-//     lower row was loaded as the upper row one step earlier, so it hits L1) instead of carrying cursors
-//     whose chunk-boundary reloads and row changes diverge;
-//   * NW starts with the run of 'l' moves along the last row (the text's tail beyond the pattern): every
-//     thread of the warp is in that phase at the same time and, for pairs of equal shape, crosses chunk
-//     boundaries in the same iteration, so it gets a tight loop on two register-resident field strings;
-//   * SW starts from the end cell the fill kernel's epilogue already found (FillArgs::endcell);
+// iteration somewhere in the warp, so every iteration runs the same code:
+//   * NW walks one DP row per iteration (row_walk.h, shared with the CPU harness of the tests): both rows
+//     are re-sought at the current column, then a branch-free scan over a window of up to 8 columns finds
+//     where the row's run of 'l' moves ends and takes the terminal 'M' or 'D'.  A config-2 path is a
+//     staircase (~150 climbs, runs of ~4.5 'l' moves), so this takes ~190 iterations per warp where a step
+//     per cell took ~690 (the run along the last row is just the first row of the loop);
+//   * SW takes one uniform branch-free step per cell (local paths are mostly diagonal, a row walk saves
+//     nothing): both rows are re-sought every step (the chunk of the lower row was loaded as the upper row
+//     one step earlier, so it hits L1) instead of carrying cursors whose chunk-boundary reloads and row
+//     changes diverge; it starts from the end cell the fill kernel's epilogue already found (FillArgs::endcell);
 //   * border tails are emitted in bulk.
 // The generic cursor walkers in b2a_format.h stay the executable specification (CPU host model, wide32 warp walker).
 #pragma once
@@ -21,6 +23,7 @@
 #include <stdint.h>
 #include "b2a_format.h"
 #include "short16_fill.cuh"
+#include "row_walk.h"
 
 namespace b2a {
 
@@ -54,6 +57,17 @@ struct DevLoader {
     }
     __device__ __forceinline__ void prefetch(uint64_t idx) const {
         asm volatile("prefetch.global.L2 [%0];" :: "l"(base + idx));
+    }
+};
+
+// row_walk.h's memory interface: read-only chunk and aligned text-word loads
+struct DevMem {
+    __device__ __forceinline__ Chunk chunk(const Chunk* p) const {
+        const uint4 v = __ldg(reinterpret_cast<const uint4*>(p));
+        return Chunk{v.x, v.y, v.z, v.w};
+    }
+    __device__ __forceinline__ uint64_t word8(const uint8_t* p) const {
+        return __ldg(reinterpret_cast<const unsigned long long*>(p));
     }
 };
 
@@ -117,99 +131,47 @@ short16_traceback_kernel(const TbArgs A)
     const uint8_t* __restrict__ T = A.txt + A.txt_off[pair];
     const int gap = A.gap, match = A.match, mismatch = A.mismatch;
     const uint32_t mh = pp_dim(d.m, half), nh = pp_dim(d.n, half);   // this pair's own shape; the record is laid out for max(n)
-    S16View<K> v{A.codes + A.code_off[pp], num_chunks(pp_max(d.n), FM::CS), (uint32_t)A.R, (uint32_t)short16_rmagic(A.R), 32u * (uint32_t)A.R,
-                 half ? 0x7632u : 0x5410u, half ? 0x4432u : 0x4410u, gap};
-    uint32_t* out = A.ops ? A.ops + A.ops_off[pair] : nullptr;
-
-    uint32_t i, j, nops = 0, word = 0, fill = 0, wpos = 0;
-    int cur = 0, best = 0;
-    const bool hw4 = !LOCAL && A.tie_hw4 != 0;
-    uint32_t mism = 0;                                    // hw4: 'M' columns whose bases differ
+    OpsRunSink sink(A.ops ? A.ops + A.ops_off[pair] : nullptr);
     PairResult res;
     res.path = 1;
-    auto put = [&](uint32_t op) {
-        word |= op << (2u * fill);
-        if (++fill == 16u) { if (out) out[wpos] = word; ++wpos; word = 0; fill = 0; }
-    };
-    auto put_run = [&](uint32_t op, uint32_t cnt) {
-        while (cnt) {
-            const uint32_t take = min(cnt, 16u - fill);
-            if (op) word |= ((op * 0x55555555u) & (take == 16u ? 0xFFFFFFFFu : ((1u << (2u * take)) - 1u))) << (2u * fill);
-            fill += take; cnt -= take;
-            if (fill == 16u) { if (out) out[wpos] = word; ++wpos; word = 0; fill = 0; }
-        }
-    };
 
-    if (LOCAL) {
-        const int4 e = A.endcell[pair];
-        res.score = e.x; res.end_i = (uint32_t)e.y; res.end_j = (uint32_t)e.z;
-        i = res.end_i; j = res.end_j;
-        if (e.x == 0) { i = 0; j = 0; }                   // hw2.cpp:202-203: best cell stays (0,0), empty alignment
-    } else {
-        i = mh; j = nh;
-        res.end_i = i; res.end_j = j;
-        int H, D;
-        v.cell(i, j, H, D);
-        res.score = H - A.bias;                           // hw2.cpp:186
-        // ---- phase A: the run of 'l' moves along the last row (hw2.cpp:146-153 on every cell of the run) ----
-        if (i >= 2u) {
-            uint32_t La, Lb;
-            const Chunk* ra = v.row_base(i, La);
-            const Chunk* rb = v.row_base(i - 1u, Lb);
-            uint32_t qa = j + La, qb = j + Lb;
-            uint32_t ca = qa / (uint32_t)FM::CS, cb = qb / (uint32_t)FM::CS;
-            int offa = K * (FM::CS - 1 - (int)(qa - ca * FM::CS)), offb = K * (FM::CS - 1 - (int)(qb - cb * FM::CS));
-            int anchor, Ha = H, Hb, Db;
-            uint64_t Xa = v.unpack(__ldg(reinterpret_cast<const uint4*>(ra + (size_t)ca * v.stride)), anchor);
-            v.cell(i - 1u, j, Hb, Db);
-            uint64_t Xb = v.unpack(__ldg(reinterpret_cast<const uint4*>(rb + (size_t)cb * v.stride)), anchor);
-            const uint8_t pc = P[i - 1u];
-            uint32_t run = 0;
-            while (j > 0u) {
-                const int Da = (int)((uint32_t)(Xa >> offa) & FM::MASK);
-                Db = (int)((uint32_t)(Xb >> offb) & FM::MASK);
-                const int Hl = Ha - Da - gap, Hd = Hb - Db - gap;
-                const int dv = Hd + (pc == T[j - 1u] ? match : mismatch);
-                // 'l' wins iff it beats the diagonal strictly and 'u' does not beat it (hw2) / it beats 'u' strictly too (hw4)
-                const bool is_l = hw4 ? (Hl + gap > dv && Hl + gap > Hb + gap) : (Hl + gap > dv && !(Hb + gap > Hl + gap));
-                if (!is_l) break;                                          // the general walk takes over
-                Ha = Hl; Hb = Hd; --j; ++run;
-                offa += K; offb += K;
-                if (offa == FM::K * FM::CS) { offa = 0; if (ca) { --ca; Xa = v.unpack(__ldg(reinterpret_cast<const uint4*>(ra + (size_t)ca * v.stride)), anchor); } }
-                if (offb == FM::K * FM::CS) { offb = 0; if (cb) { --cb; Xb = v.unpack(__ldg(reinterpret_cast<const uint4*>(rb + (size_t)cb * v.stride)), anchor); } }
-            }
-            put_run(OP_I, run); nops += run;
-        }
+    if (!LOCAL) {
+        // ---- NW: one DP row per iteration (row_walk.h) ----
+        const RowWalkPair v{A.codes + A.code_off[pp], P, T, mh, nh, (uint32_t)A.R, (uint32_t)short16_rmagic(A.R), half,
+                            match, mismatch, gap, A.bias, A.tie_hw4 != 0};
+        row_walk_global<K>(v, DevMem{}, sink, res);
+        sink.flush();
+        A.results[pair] = res;
+        return;
     }
 
-    // ---- phase B: the general walk, one uniform branch-free step per cell ----
+    // ---- SW: one uniform branch-free step per cell from the fill's end cell ----
+    S16View<K> v{A.codes + A.code_off[pp], num_chunks(pp_max(d.n), FM::CS), (uint32_t)A.R, (uint32_t)short16_rmagic(A.R), 32u * (uint32_t)A.R,
+                 half ? 0x7632u : 0x5410u, half ? 0x4432u : 0x4410u, gap};
+    const int4 e = A.endcell[pair];
+    res.score = e.x; res.end_i = (uint32_t)e.y; res.end_j = (uint32_t)e.z;
+    uint32_t i = res.end_i, j = res.end_j, nops = 0;
+    if (e.x == 0) { i = 0; j = 0; }                       // hw2.cpp:202-203: best cell stays (0,0), empty alignment
+    int cur = 0, best = 0;
     while (i > 0u && j > 0u) {
         int H, D, Hu, Du;
         v.cell(i, j, H, D);
         v.cell(i > 1u ? i - 1u : 1u, j, Hu, Du);
-        if (i == 1u) { Hu = LOCAL ? 0 : A.bias + (int)j * gap; Du = LOCAL ? -gap : 0; }     // border row, hw2.cpp:131-136 / :196-197
-        if (LOCAL && H == 0) break;                                                          // hw2.cpp:239
-        const int Hl = H - D - gap, Hd = Hu - Du - gap;
+        if (i == 1u) { Hu = 0; Du = -gap; }                                                  // border row, hw2.cpp:196-197
+        if (H == 0) break;                                                                   // hw2.cpp:239
+        const int Hd = Hu - Du - gap;
         const uint8_t pc = P[i - 1u];
         const bool eq = pc == T[j - 1u];
-        const int dv = Hd + (eq ? match : mismatch);                                         // hw2.cpp:142 / :208
-        uint32_t op;
-        if (LOCAL) op = H == dv ? OP_M : (H == Hu + gap ? OP_D : OP_I);                      // hw2.cpp:214-222 (H != 0 here)
-        else if (!hw4) { op = OP_M; int val = dv; if (Hl + gap > val) { val = Hl + gap; op = OP_I; } if (Hu + gap > val) op = OP_D; }   // hw2.cpp:145-153
-        else { op = OP_M; int val = dv; if (Hu + gap > val) { val = Hu + gap; op = OP_D; } if (Hl + gap > val) op = OP_I; }            // hw4.cpp:37-46
-        mism += (op == OP_M && !eq);
+        const int dv = Hd + (eq ? match : mismatch);                                         // hw2.cpp:208
+        const uint32_t op = H == dv ? OP_M : (H == Hu + gap ? OP_D : OP_I);                  // hw2.cpp:214-222 (H != 0 here)
         cur = (op == OP_M && eq && pc != (uint8_t)'-') ? cur + 1 : 0;                        // hw2.cpp:267-278
         best = max(best, cur);
         i -= op != OP_I; j -= op != OP_D;
-        put(op); ++nops;
+        sink.put(op); ++nops;
     }
-    if (!LOCAL) {
-        put_run(OP_D, i); nops += i; i = 0;                                                  // column 0 holds 'u' (hw2.cpp:128)
-        put_run(OP_I, j); nops += j; j = 0;                                                  // row 0 holds 'l'    (hw2.cpp:134)
-    }
-    if (fill && out) out[wpos] = word;
+    sink.flush();
     res.start_i = i; res.start_j = j; res.n_ops = nops;
-    res.overlap = hw4 ? (int)(nops - (mh + nh - nops) + mism) : best;      // gap columns = n_ops - M columns, M columns = m + n - n_ops
+    res.overlap = best;
     A.results[pair] = res;
 }
 
