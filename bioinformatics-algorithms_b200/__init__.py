@@ -21,6 +21,7 @@ HW3_BIN = os.path.join(HERE, "bin", "hw3")
 HW4_BIN = os.path.join(HERE, "bin", "hw4")
 
 GLOBAL, LOCAL = 0, 1
+SEMIGLOBAL = 2          # the whole pattern against its best-fitting substring of the text (include/b2align.h)
 SCORE_ONLY = 2
 TIE_HW4 = 4
 OPT_LANES, OPT_SEG_PAIRS, OPT_SEG_BYTES, OPT_SEG_FIRST, OPT_CKPT_BYTES, OPT_CKPT_GROUP, OPT_CKPT_COLS = 1, 2, 3, 5, 6, 7, 8
@@ -467,6 +468,11 @@ class Engine:
 
     def localAlignmentSmithWaterman(self, patterns, references, matchScore, mismatchScore, gapPenalty):
         return self._one(LOCAL, patterns, references, matchScore, mismatchScore, gapPenalty)
+
+    def semiGlobalAlignment(self, pattern, reference, matchScore, mismatchScore, gapPenalty):
+        """Semi-global mode (not in the reference): the whole pattern against the substring of the reference that suits it best;
+        record.end_j / record.start_j give where it sits (alignedReference covers reference[start_j:end_j])."""
+        return self._one(SEMIGLOBAL, pattern, reference, matchScore, mismatchScore, gapPenalty)
 
 
 def center_star_phylip(names, seqs, centre, ops):

@@ -97,7 +97,7 @@ struct WideState {
     DevBuf<WideTask> d_tasks;
     DevBuf<Chunk> d_codes;
     DevBuf<uint64_t> d_bound;                     // tagged boundary entries (wide32.cuh)
-    DevBuf<int32_t> d_final;
+    DevBuf<int32_t> d_final, d_final_col;         // per wide pair: H at the end cell; semi-global mode: also its column j*
     DevBuf<uint32_t> d_rowbest, d_progress;       // d_progress[0] is the ticket counter
     // pairs whose full record would exceed the budget: score pass with checkpoint rows, then band groups re-filled bottom-up (wide_ckpt_run)
     struct CkptSpec { uint32_t pair, m, n; uint64_t pat_off, txt_off; };
@@ -119,7 +119,7 @@ struct WideState {
         return e;
     }
     void release() {
-        d_pairs.release(); d_tasks.release(); d_codes.release(); d_bound.release(); d_final.release();
+        d_pairs.release(); d_tasks.release(); d_codes.release(); d_bound.release(); d_final.release(); d_final_col.release();
         d_rowbest.release(); d_progress.release(); d_ck.release(); d_walk.release();
     }
 };
@@ -326,34 +326,38 @@ void alpha_from_mask(AlphaInfo& a) {
 // two launches per class: the 4-symbol kernel for the pair-pairs the segment's table symbols cover, the 8-symbol kernel for the flagged
 // rest (its grid leaves at once when the segment has no fifth pattern symbol)
 template <int R, int K>
-cudaError_t launch_fill_rk(bool local, const FillArgs& a, cudaStream_t st) {
+cudaError_t launch_fill_rk(int mode, const FillArgs& a, cudaStream_t st) {
     const unsigned grid = (a.n_pp + FILL_WARPS - 1) / FILL_WARPS;
-    if (local) { short16_fill_kernel<R, K, true, false><<<grid, FILL_WARPS * 32, 0, st>>>(a); short16_fill_kernel<R, K, true, true><<<grid, FILL_WARPS * 32, 0, st>>>(a); }
+    const bool local = mode == B2A_MODE_LOCAL;
+    if (mode == B2A_MODE_SEMIGLOBAL) {
+        short16_fill_kernel<R, K, false, false, true><<<grid, FILL_WARPS * 32, 0, st>>>(a);
+        short16_fill_kernel<R, K, false, true, true><<<grid, FILL_WARPS * 32, 0, st>>>(a);
+    } else if (local) { short16_fill_kernel<R, K, true, false><<<grid, FILL_WARPS * 32, 0, st>>>(a); short16_fill_kernel<R, K, true, true><<<grid, FILL_WARPS * 32, 0, st>>>(a); }
     else { short16_fill_kernel<R, K, false, false><<<grid, FILL_WARPS * 32, 0, st>>>(a); short16_fill_kernel<R, K, false, true><<<grid, FILL_WARPS * 32, 0, st>>>(a); }
     return cudaGetLastError();
 }
 template <int K>
-cudaError_t launch_fill_k(int R, bool local, const FillArgs& a, cudaStream_t st) {
+cudaError_t launch_fill_k(int R, int mode, const FillArgs& a, cudaStream_t st) {
     switch (R) {
-        case 1: return launch_fill_rk<1, K>(local, a, st);
-        case 2: return launch_fill_rk<2, K>(local, a, st);
-        case 3: return launch_fill_rk<3, K>(local, a, st);
-        case 4: return launch_fill_rk<4, K>(local, a, st);
-        case 5: return launch_fill_rk<5, K>(local, a, st);
-        case 6: return launch_fill_rk<6, K>(local, a, st);
-        case 7: return launch_fill_rk<7, K>(local, a, st);
-        case 8: return launch_fill_rk<8, K>(local, a, st);
-        case 10: return launch_fill_rk<10, K>(local, a, st);
-        case 12: return launch_fill_rk<12, K>(local, a, st);
-        case 16: return launch_fill_rk<16, K>(local, a, st);
+        case 1: return launch_fill_rk<1, K>(mode, a, st);
+        case 2: return launch_fill_rk<2, K>(mode, a, st);
+        case 3: return launch_fill_rk<3, K>(mode, a, st);
+        case 4: return launch_fill_rk<4, K>(mode, a, st);
+        case 5: return launch_fill_rk<5, K>(mode, a, st);
+        case 6: return launch_fill_rk<6, K>(mode, a, st);
+        case 7: return launch_fill_rk<7, K>(mode, a, st);
+        case 8: return launch_fill_rk<8, K>(mode, a, st);
+        case 10: return launch_fill_rk<10, K>(mode, a, st);
+        case 12: return launch_fill_rk<12, K>(mode, a, st);
+        case 16: return launch_fill_rk<16, K>(mode, a, st);
     }
     return cudaErrorInvalidValue;
 }
-cudaError_t launch_fill(int K, int R, bool local, const FillArgs& a, cudaStream_t st) {
+cudaError_t launch_fill(int K, int R, int mode, const FillArgs& a, cudaStream_t st) {
     switch (K) {
-        case 2: return launch_fill_k<2>(R, local, a, st);
-        case 4: return launch_fill_k<4>(R, local, a, st);
-        case 8: return launch_fill_k<8>(R, local, a, st);
+        case 2: return launch_fill_k<2>(R, mode, a, st);
+        case 4: return launch_fill_k<4>(R, mode, a, st);
+        case 8: return launch_fill_k<8>(R, mode, a, st);
     }
     return cudaErrorInvalidValue;
 }
@@ -366,11 +370,23 @@ void set_kernel_attributes() {
     cudaFuncSetAttribute(short16_traceback_kernel<4, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
     cudaFuncSetAttribute(short16_traceback_kernel<8, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
     cudaFuncSetAttribute(short16_traceback_kernel<8, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
+    cudaFuncSetAttribute(short16_traceback_kernel<2, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
+    cudaFuncSetAttribute(short16_traceback_kernel<4, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
+    cudaFuncSetAttribute(short16_traceback_kernel<8, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
     cudaGetLastError();
 }
-cudaError_t launch_tb(int K, bool local, const TbArgs& a, cudaStream_t st) {
+cudaError_t launch_tb(int K, int mode, const TbArgs& a, cudaStream_t st) {
     const unsigned threads = TB_THREADS, grid = (2u * a.n_pp + threads - 1) / threads;
-    switch (K * 2 + (local ? 1 : 0)) {
+    if (mode == B2A_MODE_SEMIGLOBAL) {
+        switch (K) {
+            case 2: short16_traceback_kernel<2, false, true><<<grid, threads, 0, st>>>(a); break;
+            case 4: short16_traceback_kernel<4, false, true><<<grid, threads, 0, st>>>(a); break;
+            case 8: short16_traceback_kernel<8, false, true><<<grid, threads, 0, st>>>(a); break;
+            default: return cudaErrorInvalidValue;
+        }
+        return cudaGetLastError();
+    }
+    switch (K * 2 + (mode == B2A_MODE_LOCAL ? 1 : 0)) {
         case 4:  short16_traceback_kernel<2, false><<<grid, threads, 0, st>>>(a); break;
         case 5:  short16_traceback_kernel<2, true><<<grid, threads, 0, st>>>(a); break;
         case 8:  short16_traceback_kernel<4, false><<<grid, threads, 0, st>>>(a); break;
@@ -407,6 +423,26 @@ cudaError_t launch_wide_fill_keepcol(bool local, bool alpha4, const WideArgs& a,
                  else wide32_fill_kernel<2, false, false, false, true><<<grid, WIDE_WARPS * 32, 0, st>>>(a); }
     return cudaGetLastError();
 }
+// semi-global: whole pairs only (no KEEPCOL pass, see wide_plan)
+template <int K>
+cudaError_t launch_wide_fill_semi_k(bool store, bool alpha4, const WideArgs& a, unsigned grid, cudaStream_t st) {
+    if (!store && K != 2) return cudaErrorInvalidValue;        // score-only kernels exist for K = 2 only
+    if (store) { if (alpha4) wide32_fill_kernel<K, false, true, true, false, true><<<grid, WIDE_WARPS * 32, 0, st>>>(a);
+                 else wide32_fill_kernel<K, false, true, false, false, true><<<grid, WIDE_WARPS * 32, 0, st>>>(a); }
+    else       { if (alpha4) wide32_fill_kernel<2, false, false, true, false, true><<<grid, WIDE_WARPS * 32, 0, st>>>(a);
+                 else wide32_fill_kernel<2, false, false, false, false, true><<<grid, WIDE_WARPS * 32, 0, st>>>(a); }
+    return cudaGetLastError();
+}
+cudaError_t launch_wide_fill_semi(int K, bool store, bool alpha4, const WideArgs& a, unsigned grid, cudaStream_t st) {
+    switch (K) {
+        case 2:  return launch_wide_fill_semi_k<2>(store, alpha4, a, grid, st);
+        case 4:  return launch_wide_fill_semi_k<4>(store, alpha4, a, grid, st);
+        case 8:  return launch_wide_fill_semi_k<8>(store, alpha4, a, grid, st);
+        case 16: return launch_wide_fill_semi_k<16>(store, alpha4, a, grid, st);
+        case 32: return launch_wide_fill_semi_k<32>(store, alpha4, a, grid, st);
+    }
+    return cudaErrorInvalidValue;
+}
 cudaError_t launch_wide_fill(int K, bool local, bool store, bool alpha4, const WideArgs& a, unsigned grid, cudaStream_t st) {
     switch (K) {
         case 2:  return launch_wide_fill_k<2>(local, store, alpha4, a, grid, st);
@@ -417,9 +453,20 @@ cudaError_t launch_wide_fill(int K, bool local, bool store, bool alpha4, const W
     }
     return cudaErrorInvalidValue;
 }
-cudaError_t launch_wide_tb(int K, bool local, const WideTbArgs& a, cudaStream_t st) {
+cudaError_t launch_wide_tb(int K, int mode, const WideTbArgs& a, cudaStream_t st) {
     const unsigned threads = WIDE_TB_WARPS * 32, grid = (a.n_wide + WIDE_TB_WARPS - 1) / WIDE_TB_WARPS;
-    switch (K * 2 + (local ? 1 : 0)) {
+    if (mode == B2A_MODE_SEMIGLOBAL) {
+        switch (K) {
+            case 2:  wide32_traceback_kernel<2, false, true><<<grid, threads, 0, st>>>(a); break;
+            case 4:  wide32_traceback_kernel<4, false, true><<<grid, threads, 0, st>>>(a); break;
+            case 8:  wide32_traceback_kernel<8, false, true><<<grid, threads, 0, st>>>(a); break;
+            case 16: wide32_traceback_kernel<16, false, true><<<grid, threads, 0, st>>>(a); break;
+            case 32: wide32_traceback_kernel<32, false, true><<<grid, threads, 0, st>>>(a); break;
+            default: return cudaErrorInvalidValue;
+        }
+        return cudaGetLastError();
+    }
+    switch (K * 2 + (mode == B2A_MODE_LOCAL ? 1 : 0)) {
         case 4:  wide32_traceback_kernel<2, false><<<grid, threads, 0, st>>>(a); break;
         case 5:  wide32_traceback_kernel<2, true><<<grid, threads, 0, st>>>(a); break;
         case 8:  wide32_traceback_kernel<4, false><<<grid, threads, 0, st>>>(a); break;
@@ -455,6 +502,11 @@ int wide_plan(b2a_ctx* ctx, const uint64_t* pat_off, const uint64_t* txt_off, bo
         p.top_off = WIDE_NO_TOP; p.left_off = WIDE_NO_TOP;
         if (p.nbands >= (1u << 20)) return fail(ctx, B2A_ERR_RANGE, "wide32: pattern too long (band index must fit 20 bits)");
         if (store && (uint64_t)p.nbands * WIDE_R * num_chunks(p.n, CS, wide_skew(W.K)) * 32u * sizeof(Chunk) > ctx->wide_ckpt_bytes) {
+            // the checkpointed walk (wide_ckpt_run) has global and local borders only
+            for (uint32_t r = 0; r < ctx->n_runs; ++r)
+                if (ctx->run[r].mode == B2A_MODE_SEMIGLOBAL)
+                    return fail(ctx, B2A_ERR_RANGE, "semi-global mode: a pair whose traceback record exceeds B2A_OPT_CKPT_BYTES (the checkpointed "
+                                                    "path) is not supported; raise the option or align the pair in global or local mode");
             W.ckpt_pairs.push_back(WideState::CkptSpec{k, p.m, p.n, p.pat_off, p.txt_off});   // too large to keep: served one by one from checkpoints
             continue;
         }
@@ -473,7 +525,7 @@ int wide_plan(b2a_ctx* ctx, const uint64_t* pat_off, const uint64_t* txt_off, bo
     for (uint32_t b = 0; b < max_bands; ++b)
         for (uint32_t i : order) { if (W.pairs[i].nbands <= b) break; W.tasks.push_back(WideTask{i, b}); }
     CU(W.d_pairs.reserve(W.pairs.size())); CU(W.d_tasks.reserve(W.tasks.size()));
-    CU(W.d_codes.reserve(W.chunks)); CU(W.d_final.reserve(W.pairs.size()));
+    CU(W.d_codes.reserve(W.chunks)); CU(W.d_final.reserve(W.pairs.size())); CU(W.d_final_col.reserve(W.pairs.size()));
     CU(W.d_rowbest.reserve(W.rowbest_words)); CU(W.d_progress.reserve(1));
     // the vectors outlive the copies: every caller synchronises `st` before the next batch touches them
     if (!W.pairs.empty()) CU(cudaMemcpyAsync(W.d_pairs.p, W.pairs.data(), W.pairs.size() * sizeof(WidePair), cudaMemcpyHostToDevice, st));
@@ -494,14 +546,15 @@ int wide_fill(b2a_ctx* ctx, int r, cudaStream_t st, uint64_t* launches)
     a.pat = ctx->d_pat.p; a.txt = ctx->d_txt.p; a.pairs = W.d_pairs.p; a.tasks = W.d_tasks.p;
     a.n_tasks = (uint32_t)W.tasks.size(); a.ticket = W.d_progress.p;
     a.codes = W.d_codes.p; a.bound = W.d_bound.p; a.rowbest = W.d_rowbest.p;
-    a.final_score = W.d_final.p;
+    a.final_score = W.d_final.p; a.final_col = W.d_final_col.p;
     a.ck = nullptr;
     a.match = prm.match; a.mismatch = prm.mismatch; a.gap = prm.gap;
     a.radix = W.K < 32 ? (1u << W.K) : 0u;
     a.alpha = ctx->d_alpha.p + (ctx->alpha_slots - 1);
     const unsigned need = (unsigned)((W.tasks.size() + WIDE_WARPS - 1) / WIDE_WARPS);
     const unsigned grid = std::min<unsigned>(need, (unsigned)ctx->sm_count * 8u);
-    CU(launch_wide_fill(W.store ? W.K : 2, ctx->run[r].mode == B2A_MODE_LOCAL, W.store, W.alpha4, a, grid, st));   // score-only: no record, one instance
+    if (ctx->run[r].mode == B2A_MODE_SEMIGLOBAL) CU(launch_wide_fill_semi(W.store ? W.K : 2, W.store, W.alpha4, a, grid, st));
+    else CU(launch_wide_fill(W.store ? W.K : 2, ctx->run[r].mode == B2A_MODE_LOCAL, W.store, W.alpha4, a, grid, st));   // score-only: no record, one instance
     ++*launches;
     return B2A_OK;
 }
@@ -513,13 +566,13 @@ int wide_traceback(b2a_ctx* ctx, int r, cudaStream_t st, uint64_t* launches, boo
     const b2a_params& prm = ctx->prm;
     WideTbArgs a{};
     a.pat = ctx->d_pat.p; a.txt = ctx->d_txt.p; a.pairs = W.d_pairs.p; a.n_wide = (uint32_t)W.pairs.size();
-    a.codes = W.d_codes.p; a.rowbest = W.d_rowbest.p; a.final_score = W.d_final.p;
+    a.codes = W.d_codes.p; a.rowbest = W.d_rowbest.p; a.final_score = W.d_final.p; a.final_col = W.d_final_col.p;
     a.results = ctx->run[r].d_results.p;
     a.ops = (prm.flags & B2A_WANT_OPS) && !score_only ? ctx->run[r].d_ops.p : nullptr;
     a.ops_off = ctx->d_ops_off.p;
     a.match = prm.match; a.mismatch = prm.mismatch; a.gap = prm.gap; a.score_only = score_only ? 1 : 0;
     a.opt = (prm.flags & B2A_TIE_HW4) ? 4 : 0;
-    CU(launch_wide_tb(W.K, ctx->run[r].mode == B2A_MODE_LOCAL, a, st));
+    CU(launch_wide_tb(W.K, ctx->run[r].mode, a, st));
     ++*launches;
     return B2A_OK;
 }
@@ -716,7 +769,7 @@ int launch_segment(b2a_ctx* ctx, size_t si, int r, uint64_t* launches)
         a.dirty = ctx->d_dirty.p + sg.pp_first + c.first;
         a.dirty_list = ctx->d_dirty_list.p + sg.pp_first + c.first;
         a.dirty_cnt = ctx->d_dirty_cnt.p + si * DIRTY_CLASSES + ci;
-        CU(launch_fill(ctx->K, c.R, local, a, st));
+        CU(launch_fill(ctx->K, c.R, mode, a, st));
         *launches += 2;
     }
     CU(cudaEventRecord(ev[2], st));
@@ -737,7 +790,7 @@ int launch_segment(b2a_ctx* ctx, size_t si, int r, uint64_t* launches)
         a.tie_hw4 = (prm.flags & B2A_TIE_HW4) ? 1 : 0;
         a.alpha = alpha;
         a.dirty = ctx->d_dirty.p + sg.pp_first + c.first;
-        CU(launch_tb(ctx->K, local, a, st));
+        CU(launch_tb(ctx->K, mode, a, st));
         ++*launches;
     }
     CU(cudaEventRecord(ev[3], st));
@@ -933,7 +986,7 @@ int batch_prepare(b2a_ctx* ctx, const b2a_params* prms, uint32_t n_runs, const u
     bool any_local = false;
     for (uint32_t r = 0; r < n_runs; ++r) {
         const b2a_params& q = prms[r];
-        if (q.mode != B2A_MODE_GLOBAL && q.mode != B2A_MODE_LOCAL) return fail(ctx, B2A_ERR_ARG, "b2a_batch_upload: bad mode");
+        if (q.mode != B2A_MODE_GLOBAL && q.mode != B2A_MODE_LOCAL && q.mode != B2A_MODE_SEMIGLOBAL) return fail(ctx, B2A_ERR_ARG, "b2a_batch_upload: bad mode");
         if ((q.flags & B2A_TIE_HW4) && q.mode != B2A_MODE_GLOBAL) return fail(ctx, B2A_ERR_ARG, "B2A_TIE_HW4 applies to the global mode only");
         if (q.match != prm->match || q.mismatch != prm->mismatch || q.gap != prm->gap || ((q.flags ^ prm->flags) & ~B2A_TIE_HW4))
             return fail(ctx, B2A_ERR_ARG, "b2a_align_batch_multi: the runs of one batch share scoring and flags (they differ in mode)");
@@ -1010,7 +1063,7 @@ int batch_prepare(b2a_ctx* ctx, const b2a_params* prms, uint32_t n_runs, const u
     for (uint32_t r = 0; r < n_runs; ++r) {
         RunBuf& rb = ctx->run[r];
         CU(rb.d_results.reserve(n_pairs));
-        if (rb.mode == B2A_MODE_LOCAL) CU(rb.d_endcell.reserve(n_pairs));
+        if (rb.mode != B2A_MODE_GLOBAL) CU(rb.d_endcell.reserve(n_pairs));    // the short16 fill epilogues' end cells (local, semi-global)
         if (want_ops) CU(rb.d_ops.reserve(ops_bound));
     }
     CU(ctx->d_alpha.reserve(ctx->alpha_slots)); CU(ctx->h_alpha.reserve(ctx->alpha_slots));
@@ -1137,7 +1190,8 @@ int batch_prepare(b2a_ctx* ctx, const b2a_params* prms, uint32_t n_runs, const u
             else pending[last_key] = last_idx;
         }
         // Leftovers (one per distinct shape): zip pairs of DIFFERENT shapes, neighbours in (rows per lane, n, m) order so that little
-        // is padded.  Safe for NW always (the score is read at the true end cell); for SW the junk columns of the shorter text must
+        // is padded.  Safe for NW always (the score is read at the true end cell) and for semi-global mode (its epilogue scans only
+        // the pair's own row m, columns 0..n, and its walk only the pair's own cells); for SW the junk columns of the shorter text must
         // stay strictly below the real maximum, which needs gap < 0 and mismatch < 0.  What still has no partner runs as a singleton
         // (both halves carry the same pair).
         {

@@ -118,7 +118,11 @@ B2A_HD int short16_R(uint32_t m) {
     const int r = (int)((m + 31u) / 32u);
     return r <= 8 ? r : (r <= 10 ? 10 : (r <= 12 ? 12 : 16));
 }
+// mode: 0 global, 1 local, 2 semi-global.  Semi-global takes the global plan: with gap <= 0 every semi-global H lies in
+// i*gap <= H(i,j) <= min(i,j)*max(match,0), inside the range the global bias and checks already cover, and its fill (H space,
+// table scores s) needs no more than the global fill (S space, scores s - 2 gap), so one plan serves every run of a batch.
 B2A_HD bool short16_plan(int mode, uint32_t m, uint32_t n, int match, int mismatch, int gap, Short16Plan& pl) {
+    if (mode == 2) mode = 0;
     if (m == 0 || n == 0 || m > 32u * SHORT16_MAX_R || n > 30000u) return false;     // (the int16 range test below is the real limit on n)
     pl.K = delta_bits(match, mismatch, gap);
     if (pl.K == 0) return false;

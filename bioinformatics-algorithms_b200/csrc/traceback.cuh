@@ -36,7 +36,7 @@ struct TbArgs {
     const uint64_t* code_off;
     const Chunk*    codes;
     const uint32_t* rowbest;
-    const int4*     endcell;    // local mode, per pair: {score, end_i, end_j, 0} from the fill kernel
+    const int4*     endcell;    // local and semi-global modes, per pair: {score, end_i, end_j, 0} from the fill kernel
     PairResult*     results;    // indexed by pair
     uint32_t*       ops;        // packed 2-bit ops, may be null
     const uint64_t* ops_off;    // per pair word offset into ops
@@ -115,7 +115,8 @@ struct S16View {
 #ifndef TB_MIN_CTAS
 #define TB_MIN_CTAS 1
 #endif
-template <int K, bool LOCAL>
+// SEMI (with LOCAL = false): the semi-global row walk from the end cell the fill's epilogue found (FillArgs::endcell)
+template <int K, bool LOCAL, bool SEMI = false>
 __global__ void __launch_bounds__(TB_THREADS, TB_MIN_CTAS)
 short16_traceback_kernel(const TbArgs A)
 {
@@ -135,6 +136,15 @@ short16_traceback_kernel(const TbArgs A)
     PairResult res;
     res.path = 1;
 
+    if (SEMI) {
+        RowWalkPair v{A.codes + A.code_off[pp], P, T, mh, nh, (uint32_t)A.R, (uint32_t)short16_rmagic(A.R), half,
+                      match, mismatch, gap, A.bias, false};
+        v.j_end = (uint32_t)A.endcell[pair].z;
+        row_walk_global<K, DevMem, OpsRunSink, true>(v, DevMem{}, sink, res);
+        sink.flush();
+        A.results[pair] = res;
+        return;
+    }
     if (!LOCAL) {
         // ---- NW: one DP row per iteration (row_walk.h) ----
         const RowWalkPair v{A.codes + A.code_off[pp], P, T, mh, nh, (uint32_t)A.R, (uint32_t)short16_rmagic(A.R), half,

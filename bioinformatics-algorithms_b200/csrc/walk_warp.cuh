@@ -73,7 +73,8 @@ __device__ __forceinline__ void warp_prefetch_window(const PairView& v, const Lo
 // (Measured and dropped in round 2: rounds that decide the cells of THREE neighbouring diagonals per lane, so that a window survives one
 //  indel and continues on the shifted diagonal.  Fewer rounds, but three seeks + three decisions per lane made a round 1.8x as expensive:
 //  the 100 kb pair of config 4 went from 7.0 to 8.0 ms.  A round is bound by its ~110 instructions per lane, not by the load latency.)
-template <class FM, class Loader, bool LOCAL>
+// SEMI (with LOCAL = false): NW decisions over the semi-global record, whose row 0 is free (H = 0, D = -gap: the cursor's SW border).
+template <class FM, class Loader, bool LOCAL, bool SEMI = false>
 __device__ __forceinline__ void warp_walk(const PairView& v, const Loader& ld, WarpOpsSink& sink, uint32_t& i, uint32_t& j,
                                            uint32_t& nops, int& best, uint32_t& mism, int& cur)
 {
@@ -87,7 +88,7 @@ __device__ __forceinline__ void warp_walk(const PairView& v, const Loader& ld, W
         uint32_t op = OP_M; bool stop = false, exact = false, differ = false;
         if (valid) {
             const uint32_t ci = i - di, cj = j - dj;
-            RowCursor<FM, Loader, LOCAL> rc, ru;
+            RowCursor<FM, Loader, LOCAL || SEMI> rc, ru;
             rc.seek(v, ld, ci, cj);
             ru.seek(v, ld, ci - 1u, cj);
             const int H = rc.H, Hl = H - rc.D() - v.gap;            // H(ci, cj-1); frozen lanes make this the border at cj == 1
